@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- UNet steps/sec of the Paint-with-Words denoising loop on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[1] -- aurora_1 colour map, SD1.5-shaped UNet (seeded random
@@ -22,6 +22,9 @@ One JSON line on stdout (rank 0):
   reference_gpu_eager   comparison only: the reference's loop and inj_forward op sequence as eager fp16 PyTorch on this GPU
   cpu_baseline  the oracle port of the reference loop on this box's host cores (rank 0, N=1 only), bounded sample
 --impl reference: only that CPU loop (the reference is pure Python/torch; its CPU path is what is timed).
+--dump-outputs DIR: after the timed steps, write the latents the last timed step left (what PwWSampler.run returns)
+as DIR/latents.npy (float32; DIR/latents_rank<r>.npy per rank when N > 1).  Inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -526,6 +529,13 @@ def _claim_stdout():
         os.dup2(2, 1)
 
 
+def dump_outputs(out_dir: str, arrays: dict, rank: int, world: int):
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), t.detach().float().cpu().numpy())
+
+
 def emit(line: dict):
     data = (json.dumps(line) + "\n").encode()
     if _REAL_STDOUT is None:
@@ -546,7 +556,13 @@ def main():
     ap.add_argument("--quick", action="store_true", help="timed region only (for ncu launch lists): no e2e/roofline/cpu legs")
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS),
                     help="BASELINE.json config (1-based); 2 = configs[1], the one the metric is quoted on (default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents of the last timed step to DIR/latents.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 arm")
     cfg = CONFIGS[args.config]
     rank, local_rank, world = sharding.env_world()
     if args.impl == "reference":
@@ -629,6 +645,8 @@ def main():
         with ClockSampler(local_rank) as clk:
             ms = timed_region(args.steps)
         clocks = clk.summary()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"latents": sampler.latents}, rank, world)
         per_step_launches = sampler.native_launches_per_step
         if per_step_launches is None:
             per_step_launches = (_native.launch_count - launches_before) // max(1, args.steps)

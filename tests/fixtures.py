@@ -1,7 +1,9 @@
 """Shared test/bench inputs rebuilt from the committed golden fixtures (no /root/reference needed)."""
+import math
 import os
 
 import numpy as np
+import torch
 from PIL import Image
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -29,6 +31,16 @@ def color_map_image(name: str, size: int = 512) -> Image.Image:
     if size != img.size[0]:
         img = img.resize((size, size), Image.NEAREST)   # gradio_pww.py:17 behaviour
     return img
+
+
+def digest(t: torch.Tensor) -> np.ndarray:
+    """[sum, sum of squares, weighted checksum] in float64 -- for tensors too big to commit.  Each sum is exactly
+    rounded (math.fsum over the non-zero entries), so the digest of the same tensor is the same on every CPU, whatever
+    its vector width or thread count."""
+    x = t.double().flatten()
+    nz = torch.nonzero(x).flatten()
+    v, w = x[nz], (nz + 1).double() % 9973
+    return np.array([math.fsum(v.tolist()), math.fsum((v * v).tolist()), math.fsum((v * w).tolist())])
 
 
 def moon_mask_image(size: int = 512) -> Image.Image:

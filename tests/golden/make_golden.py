@@ -31,6 +31,7 @@ sys.path.insert(0, ROOT)
 from oracle.ref_loader import REFERENCE_ROOT, load_reference  # noqa: E402
 from paint_with_words_sd_b200.synthetic import SimpleWordTokenizer  # noqa: E402
 from paint_with_words_sd_b200.unet import CrossAttention  # noqa: E402
+from tests.fixtures import digest  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
@@ -59,13 +60,6 @@ def region_index_map(img: Image.Image, colors) -> np.ndarray:
     for i, c in enumerate(colors):
         idx[(a == np.array(c, dtype=np.uint8)).all(-1)] = i + 1
     return idx
-
-
-def digest(t: torch.Tensor) -> np.ndarray:
-    """[sum, sum of squares, weighted checksum] in float64 -- for tensors too big to commit."""
-    x = t.double().flatten()
-    w = torch.arange(1, x.numel() + 1, dtype=torch.float64) % 9973
-    return np.array([x.sum().item(), (x * x).sum().item(), (x * w).sum().item()])
 
 
 def main():
