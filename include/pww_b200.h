@@ -159,6 +159,37 @@ int pww_geglu_f16(const void* in, void* out, int64_t M, int I, void* stream);
 int pww_add_layernorm_f16(const void* x, const void* res, const void* gamma, const void* beta, void* sum_out, void* y,
                           int64_t M, int C, float eps, void* stream);
 
+/*
+ * Sampler step of the Euler, Euler-ancestral and DPM-Solver++(2M) schedulers (paint_with_words_sd_b200/scheduler.py),
+ * around the UNet forward of one denoising step of m images.  Each of them updates the latents as
+ *     eps = eps_u + g * (eps_c - eps_u),  x0 = x - sigma * eps,
+ *     x'  = a * x + b * eps + c * x0 + d * x0_prev + s * xi,  x0_prev <- x0
+ * with per-step scalars read from a DEVICE coefficient row `coef` of 12 fp32 (so a CUDA graph replays each step with
+ * new values after a copy into the row):
+ *     coef[0] sigma   coef[1] c_in = 1/sqrt(sigma^2+1)   coef[2] UNet timestep   coef[3..7] a, b, c, d, s
+ *     coef[8] G(sigma) (read by the attention path)   coef[9] absolute step index (for the noise)   coef[10..11] unused
+ * Latent-shaped fp32 tensors are NCHW contiguous.
+ */
+
+/* UNet input of a step: out [2m, C+Ce, H, W] fp16 CHANNELS-LAST (element (n,c,y,x) at ((n*H + y)*W + x)*(C+Ce) + c),
+ * rows n and n+m both = cat(c_in * latents[n], extra[n]) rounded to fp16.  latents [m, C, H, W] fp32; extra
+ * [m, Ce, H, W] fp32 (e.g. the inpaint mask and masked-image latents), NULL iff Ce == 0.  C + Ce <= 16. */
+int pww_sampler_prepare_f16(const float* latents, const float* extra, const float* coef, void* out,
+                            int m, int C, int Ce, int H, int W, void* stream);
+
+/* CFG combine + sampler update.  eps: the UNet output [2m, C, H, W] fp16 (cond rows 0..m-1, uncond rows m..2m-1) at
+ * the given element strides (any layout, e.g. channels-last).  latents and x0_prev [m, C, H, W] fp32 are updated in
+ * place.  seeds [m]: the noise seed of each image; xi is pww_randn_f32(seed, step) of that image (drawn only when
+ * coef[7] != 0). */
+int pww_sampler_step_f32(const void* eps, int64_t eps_n_stride, int64_t eps_c_stride, int64_t eps_h_stride,
+                         int64_t eps_w_stride, float* latents, float* x0_prev, const float* coef,
+                         const uint64_t* seeds, float guidance_scale, int m, int C, int H, int W, void* stream);
+
+/* n standard normals: Philox4x32-10 keyed by `seed`, counter (element / 4, step), Box-Muller.  out[e] is the noise
+ * pww_sampler_step_f32 adds to element e (NCHW index within the image) of an image with this seed at this step; it
+ * depends on nothing else (not on batch position, batch size or device). */
+int pww_randn_f32(float* out, int64_t n, uint64_t seed, int step, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -13,7 +13,9 @@ from .pipeline import (  # noqa: F401
     PaintWithWord_StableDiffusionInpaintPipeline, PaintWithWord_StableDiffusionPipeline, PwWSampler, paint_with_words,
     paint_with_words_inpaint, preprocess, prepare_mask_and_masked_image, pww_load_tools,
 )
-from .scheduler import LMSDiscreteScheduler  # noqa: F401
+from .scheduler import (  # noqa: F401
+    DPMSolverMultistepScheduler, EulerAncestralDiscreteScheduler, EulerDiscreteScheduler, LMSDiscreteScheduler,
+)
 from .weight_function import UnsupportedWeightFunction, WeightFunction, probe_weight_function  # noqa: F401
 
 __version__ = "0.1.0"

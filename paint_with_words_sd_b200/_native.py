@@ -19,6 +19,7 @@ EXPORTS = (
     "pww_xattn_workspace_bytes", "pww_xattn_stats_f16", "pww_xattn_fwd_f16", "pww_attn_fwd_f16",
     "pww_xattn_fused_workspace_bytes", "pww_xattn_fused_f16",
     "pww_groupnorm_workspace_bytes", "pww_groupnorm_nhwc_f16", "pww_geglu_f16", "pww_add_layernorm_f16",
+    "pww_sampler_prepare_f16", "pww_sampler_step_f32", "pww_randn_f32",
 )
 
 
@@ -68,6 +69,13 @@ def lib() -> ctypes.CDLL:
     L.pww_geglu_f16.argtypes = [c_vp, c_vp, c_i64, c_i, c_vp]
     L.pww_add_layernorm_f16.restype = c_i
     L.pww_add_layernorm_f16.argtypes = [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i, c_f, c_vp]
+    L.pww_sampler_prepare_f16.restype = c_i
+    L.pww_sampler_prepare_f16.argtypes = [c_vp, c_vp, c_vp, c_vp, c_i, c_i, c_i, c_i, c_i, c_vp]
+    L.pww_sampler_step_f32.restype = c_i
+    L.pww_sampler_step_f32.argtypes = [c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_f, c_i, c_i, c_i,
+                                       c_i, c_vp]
+    L.pww_randn_f32.restype = c_i
+    L.pww_randn_f32.argtypes = [c_vp, c_i64, ctypes.c_uint64, c_i, c_vp]
     _lib = L
     return L
 

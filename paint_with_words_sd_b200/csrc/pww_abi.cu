@@ -8,6 +8,7 @@
 #include "xattn_fused2.cuh"
 #include "attn_tc.cuh"
 #include "unet_ops.cuh"
+#include "sampler.cuh"
 #include <stdlib.h>
 
 namespace {
@@ -17,6 +18,16 @@ thread_local char g_last_cuda_error[640] = "";
 int cuda_fail(cudaError_t e);
 
 bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) == 0; }
+
+// Grid of an elementwise grid-stride kernel over `work` items, 256 threads a block.
+unsigned elementwise_grid(long long work) {
+  long long blocks = (work + 255) / 256;
+  const long long cap = (long long)pww::tc::num_sms() * 8;
+  if (blocks > cap) blocks = cap;
+  return (unsigned)(blocks < 1 ? 1 : blocks);
+}
 
 bool supported_head_dim(int D) { return D == 40 || D == 64 || D == 80 || D == 160; }
 
@@ -380,6 +391,64 @@ int pww_attn_fwd_f16(const void* q, const void* k, const void* v, void* out, int
     case 80: e = pww::fa::launch<80>(q, k, v, out, B, H, N, qkv_batch_stride, qkv_row_stride, o_batch_stride, o_row_stride, scale, s); break;
     case 160: e = pww::fa::launch<160>(q, k, v, out, B, H, N, qkv_batch_stride, qkv_row_stride, o_batch_stride, o_row_stride, scale, s); break;
   }
+  return e == cudaSuccess ? PWW_OK : cuda_fail(e);
+}
+
+int pww_sampler_prepare_f16(const float* latents, const float* extra, const float* coef, void* out, int m, int C, int Ce,
+                            int H, int W, void* stream) {
+  if (!latents || !coef || !out || m <= 0 || C <= 0 || Ce < 0 || H <= 0 || W <= 0) return PWW_ERR_BAD_ARG;
+  if ((Ce > 0) != (extra != nullptr)) return PWW_ERR_BAD_ARG;
+  if (!aligned4(latents) || !aligned4(coef) || (extra && !aligned4(extra)) || (reinterpret_cast<uintptr_t>(out) & 1u))
+    return PWW_ERR_BAD_ARG;
+  const int Ct = C + Ce;
+  const long long HW = (long long)H * W;
+  if (Ct > pww::smp::kMaxPrepChannels || HW > (1LL << 40) || (long long)m > (1LL << 20)) return PWW_ERR_UNSUPPORTED;
+  pww::smp::PrepareParams p;
+  p.lat = latents; p.extra = extra; p.coef = coef; p.out = (__half*)out;
+  p.m = m; p.C = C; p.Ce = Ce; p.HW = HW;
+  p.vec_in = (HW % 4) == 0 && aligned16(latents) && (!extra || aligned16(extra));
+  p.vec_out = (HW % 4) == 0 && (Ct % 2) == 0 && aligned16(out);
+  const unsigned grid = elementwise_grid((long long)m * ((HW + 3) / 4));
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (Ct) {
+#define PWW_PREP_CASE(n) case n: pww::smp::prepare_kernel<n><<<grid, 256, 0, s>>>(p); break;
+    PWW_PREP_CASE(1) PWW_PREP_CASE(2) PWW_PREP_CASE(3) PWW_PREP_CASE(4) PWW_PREP_CASE(5) PWW_PREP_CASE(6)
+    PWW_PREP_CASE(7) PWW_PREP_CASE(8) PWW_PREP_CASE(9) PWW_PREP_CASE(10) PWW_PREP_CASE(11) PWW_PREP_CASE(12)
+    PWW_PREP_CASE(13) PWW_PREP_CASE(14) PWW_PREP_CASE(15) PWW_PREP_CASE(16)
+#undef PWW_PREP_CASE
+    default: return PWW_ERR_UNSUPPORTED;
+  }
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? PWW_OK : cuda_fail(e);
+}
+
+int pww_sampler_step_f32(const void* eps, int64_t eps_n_stride, int64_t eps_c_stride, int64_t eps_h_stride,
+                         int64_t eps_w_stride, float* latents, float* x0_prev, const float* coef, const uint64_t* seeds,
+                         float guidance_scale, int m, int C, int H, int W, void* stream) {
+  if (!eps || !latents || !x0_prev || !coef || !seeds || m <= 0 || C <= 0 || H <= 0 || W <= 0) return PWW_ERR_BAD_ARG;
+  if ((reinterpret_cast<uintptr_t>(eps) & 1u) || !aligned4(latents) || !aligned4(x0_prev) || !aligned4(coef) ||
+      (reinterpret_cast<uintptr_t>(seeds) & 7u))
+    return PWW_ERR_BAD_ARG;
+  if (eps_n_stride <= 0 || eps_c_stride <= 0 || eps_h_stride <= 0 || eps_w_stride <= 0) return PWW_ERR_BAD_ARG;
+  const long long chw = (long long)C * H * W;
+  if (chw > (1LL << 40) || (long long)m > (1LL << 20)) return PWW_ERR_UNSUPPORTED;
+  pww::smp::StepParams p;
+  p.eps = (const __half*)eps;
+  p.sn = eps_n_stride; p.sc = eps_c_stride; p.sh = eps_h_stride; p.sw = eps_w_stride;
+  p.lat = latents; p.x0p = x0_prev; p.coef = coef; p.seeds = (const unsigned long long*)seeds;
+  p.guidance = guidance_scale;
+  p.m = m; p.C = C; p.H = H; p.W = W; p.chw = chw;
+  p.vec = (chw % 4) == 0 && aligned16(latents) && aligned16(x0_prev);
+  pww::smp::step_kernel<<<elementwise_grid((long long)m * ((chw + 3) / 4)), 256, 0, (cudaStream_t)stream>>>(p);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? PWW_OK : cuda_fail(e);
+}
+
+int pww_randn_f32(float* out, int64_t n, uint64_t seed, int step, void* stream) {
+  if (!out || n <= 0 || step < 0 || !aligned4(out)) return PWW_ERR_BAD_ARG;
+  if (n > (1LL << 42)) return PWW_ERR_UNSUPPORTED;
+  pww::smp::randn_kernel<<<elementwise_grid((n + 3) / 4), 256, 0, (cudaStream_t)stream>>>(out, n, seed, (uint32_t)step);
+  cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? PWW_OK : cuda_fail(e);
 }
 

@@ -8,6 +8,7 @@ What is different underneath (results equal within the stated fp16 tolerance):
     statistic instead of two batch-1 forwards (paint_with_words.py:483-499);
   * the whole step (UNet, CFG combine, LMS update) is captured in a CUDA graph; sigma, G(sigma) and the
     LMS coefficients are device scalars refreshed by tiny copies, so a replay does no host math;
+  * with the Euler, Euler-ancestral and DPM-Solver++(2M) schedulers the CFG combine and update are one native kernel;
   * K/V of the text context are step-invariant, so the context tensors are staged once per image.
 """
 from __future__ import annotations
@@ -22,7 +23,8 @@ from PIL import Image
 
 from . import attention as _attention
 from .conditioning import _encode_text_color_inputs, _get_binary_mask, pack_weight_map, packed_key
-from .scheduler import LMSDiscreteScheduler
+from . import sampler_ops as _sampler_ops
+from .scheduler import SIGMA_SAMPLERS, LMSDiscreteScheduler, _CoefficientScheduler
 from .synthetic import IdentityVAE, RandomTextEncoder, SimpleWordTokenizer
 from .unet import UNet2DConditionModel, UNetConfig, build_unet
 from .weight_function import g_of_sigma, probe_weight_function
@@ -122,13 +124,26 @@ class PwWSampler:
     """Denoising loop for a group of images on ONE GPU (paint_with_words.py:471-506 semantics per image).
 
     Each image i has a cond context dict, an uncond context dict and latents; a step runs one UNet
-    forward over the batch [cond_0..cond_{m-1}, uncond_0..uncond_{m-1}], the CFG combine and the LMS
+    forward over the batch [cond_0..cond_{m-1}, uncond_0..uncond_{m-1}], the CFG combine and the sampler
     update.  `use_graph=True` captures the step in a CUDA graph.
+
+    With `LMSDiscreteScheduler` the update is the LMS step below in PyTorch.  With the Euler, Euler-ancestral and
+    DPM-Solver++(2M) schedulers a step is "prepare -> UNet -> step": one native launch writes the fp16 channels-last
+    UNet input, one applies the CFG combine and the update (sampler_ops.py).  `noise_seeds` (one per image, default
+    0..m-1) key the ancestral noise, so an image's result does not depend on how images are batched.
     """
 
     def __init__(self, unet, scheduler: LMSDiscreteScheduler, cond_ctxs: Sequence[dict], uncond_ctxs: Sequence[dict],
                  latents: torch.Tensor, weight_function: Callable, guidance_scale: float = 7.5,
-                 extra_input: Optional[torch.Tensor] = None, use_graph: bool = True, timesteps=None):
+                 extra_input: Optional[torch.Tensor] = None, use_graph: bool = True, timesteps=None,
+                 noise_seeds: Optional[Sequence[int]] = None):
+        if isinstance(scheduler, LMSDiscreteScheduler):
+            self._fused = False
+        elif isinstance(scheduler, _CoefficientScheduler):
+            self._fused = True
+        else:
+            names = ", ".join(c.__name__ for c in (LMSDiscreteScheduler,) + SIGMA_SAMPLERS)
+            raise TypeError(f"PwWSampler does not support {type(scheduler).__name__}; supported schedulers: {names}")
         self.unet, self.scheduler = unet, scheduler
         self.m = len(cond_ctxs)
         self.device = latents.device
@@ -149,11 +164,48 @@ class PwWSampler:
         # Per-step scalars (sigma, 1/sqrt(sigma^2+1), t, 4 LMS coefficients, G(sigma)) are tabulated
         # once on the host and uploaded; a step copies its row into `_params` (one 32-byte D2D copy), so
         # a captured graph sees new values and the host never feeds the stream mid-loop.
-        self._table = self._build_step_table().to(dev)
-        self._params = torch.zeros(8, dtype=torch.float32, device=dev)
-        self._derivs = torch.zeros((4,) + tuple(self.latents.shape), dtype=torch.float32, device=dev)
-        self._ctx["G_SIGMA"] = self._params[7:8]
+        if self._fused:
+            self._init_fused(noise_seeds)
+        else:
+            self._table = self._build_step_table().to(dev)
+            self._params = torch.zeros(8, dtype=torch.float32, device=dev)
+            self._derivs = torch.zeros((4,) + tuple(self.latents.shape), dtype=torch.float32, device=dev)
+            self._ctx["G_SIGMA"] = self._params[7:8]
         self._step_no = 0
+
+    def _init_fused(self, noise_seeds):
+        if not self.latents.is_cuda:
+            raise ValueError(f"{type(self.scheduler).__name__} runs its step on the GPU; latents are on {self.device}")
+        if self._unet_dtype != torch.float16:
+            raise ValueError(f"{type(self.scheduler).__name__} feeds the UNet fp16; this UNet is {self._unet_dtype}")
+        dev, m = self.device, self.m
+        self.latents = self.latents.contiguous()
+        seeds = list(range(m)) if noise_seeds is None else [int(v) for v in noise_seeds]
+        if len(seeds) != m:
+            raise ValueError(f"noise_seeds has {len(seeds)} entries for {m} images")
+        self._seeds = torch.tensor(seeds, dtype=torch.int64, device=dev)
+        self._extra = None if self.extra_input is None else self.extra_input.to(dev, torch.float32).contiguous()
+        _, c, h, w = self.latents.shape
+        ce = 0 if self._extra is None else self._extra.shape[1]
+        self._unet_in = torch.empty((2 * m, c + ce, h, w), dtype=torch.float16, device=dev,
+                                    memory_format=torch.channels_last)
+        self._x0_prev = torch.zeros_like(self.latents)
+        self._table = self._build_coefficient_table().to(dev)
+        self._params = torch.zeros(_sampler_ops.COEF_ROW, dtype=torch.float32, device=dev)
+        self._ctx["G_SIGMA"] = self._params[8:9]
+
+    def _build_coefficient_table(self) -> torch.Tensor:
+        """Row k (run step k): sigma, c_in, t, a, b, c, d, s, G(sigma), absolute step index, 0, 0
+        (layout in include/pww_b200.h)."""
+        sch = self.scheduler
+        rows = []
+        for k, t in enumerate(self.timesteps):
+            si = sch.step_index_of(t)
+            sigma = float(sch.sigmas[si])
+            a, b, c, d, s = sch.coefficients(si, first=(k == 0))
+            g = g_of_sigma(self.weight_function, self._probed, sch.sigmas[si])
+            rows.append([sigma, 1.0 / math.sqrt(sigma * sigma + 1.0), float(t), a, b, c, d, s, g, float(si), 0.0, 0.0])
+        return torch.tensor(rows, dtype=torch.float32)
 
     def _build_step_table(self) -> torch.Tensor:
         sch = self.scheduler
@@ -207,6 +259,9 @@ class PwWSampler:
 
     # -- one step, expressed only with device tensors / device scalars --------------------------
     def _step_body(self):
+        if self._fused:
+            self._fused_step_body()
+            return
         m = self.m
         x = self.latents * self._params[1]
         if self.extra_input is not None:
@@ -220,6 +275,15 @@ class PwWSampler:
         self._derivs[0].copy_(noise_pred)
         upd = (self._params[3:7].view(4, 1, 1, 1, 1) * self._derivs).sum(0)
         self.latents.add_(upd)
+
+    def _fused_step_body(self):
+        _sampler_ops.prepare_unet_input(self.latents, self._extra, self._params, self._unet_in)
+        eps = self.unet(self._unet_in, self._params[2:3], encoder_hidden_states=self._ctx).sample
+        _sampler_ops.sampler_step(eps, self.latents, self._x0_prev, self._params, self._seeds, self.guidance_scale)
+
+    def _state(self) -> List[torch.Tensor]:
+        """Device tensors a step updates in place (what warm-up and capture must restore)."""
+        return [self.latents, self._x0_prev] if self._fused else [self.latents, self._derivs]
 
     def _set_step_scalars(self, i: int, step_index: int):
         self._params.copy_(self._table[i])
@@ -264,9 +328,9 @@ class PwWSampler:
         return n
 
     def restart(self, latents: Optional[torch.Tensor] = None):
-        """Rewind to step 0 (fresh LMS history), optionally with new latents."""
+        """Rewind to step 0 (fresh LMS / multistep history), optionally with new latents."""
         self._step_no = 0
-        self._derivs.zero_()
+        self._state()[1].zero_()
         if latents is not None:
             self.latents.copy_(latents)
 
@@ -285,21 +349,24 @@ class PwWSampler:
         self._step_no += 1
 
     def _capture(self):
-        snap = (self.latents.clone(), self._derivs.clone())
+        state = self._state()
+        snap = [t.clone() for t in state]
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(s):
             for _ in range(2):
                 self._step_body()
         torch.cuda.current_stream(self.device).wait_stream(s)
-        self.latents.copy_(snap[0]); self._derivs.copy_(snap[1])
+        for t, v in zip(state, snap):
+            t.copy_(v)
         g = torch.cuda.CUDAGraph()
         from . import _native
         before = _native.launch_count
         with torch.cuda.graph(g):
             self._step_body()
         self.native_launches_per_step = _native.launch_count - before
-        self.latents.copy_(snap[0]); self._derivs.copy_(snap[1])
+        for t, v in zip(state, snap):
+            t.copy_(v)
         self._graph = g
 
     def run(self, num_steps: Optional[int] = None) -> torch.Tensor:
@@ -355,7 +422,7 @@ def paint_with_words(
         latents = scheduler.add_noise(init_latents, noise, timesteps[:1])
 
     sampler = PwWSampler(unet, scheduler, [cond], [uncond], latents, weight_function, guidance_scale,
-                         timesteps=timesteps)
+                         timesteps=timesteps, noise_seeds=[seed])
     latents = sampler.run()
     if return_latents:
         return latents
@@ -445,7 +512,8 @@ def paint_with_words_inpaint(
             f"num_channels_latents: {latents.shape[1]} + num_channels_mask: {mask.shape[1]} + "
             f"num_channels_masked_image: {masked_image_latents.shape[1]} = {total}.")
     sampler = PwWSampler(unet, scheduler, [cond], [uncond], latents, weight_function, guidance_scale,
-                         extra_input=torch.cat([mask, masked_image_latents], 1).float(), timesteps=timesteps)
+                         extra_input=torch.cat([mask, masked_image_latents], 1).float(), timesteps=timesteps,
+                         noise_seeds=[seed])
     latents = sampler.run()
     if return_latents:
         return latents
